@@ -31,6 +31,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "training views/sec (fwd+bwd+Adam) @1M Gaussians 1080p"
 UNIT = "views/s"
@@ -56,7 +57,35 @@ def parse():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="N > 1: weak = --views-per-gpu views on every GPU; strong = the config's total view count "
                          "(8 for C3, 32 for C4) split over the GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (its loss and the parameters "
+                         "after its Adam step, a fixed seeded sample of DUMP_ROWS Gaussians) as DIR/<name>.npy, float32")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this project's training step (--impl ours)")
+    return a
+
+
+DUMP_ROWS = 65536  # 59 floats per Gaussian at SH degree 3: ~15 MB per dump
+
+
+def dump_last_step(tr, n: int, out_dir: str) -> None:
+    """Writes the loss of the last step (summed over its views) and the parameters it left behind, for the rows of a fixed
+    seeded sample of the Gaussians, so that two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+
+    torch.cuda.synchronize()
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    idx = torch.as_tensor(rows, device=tr.device)
+    out = {"loss": tr.loss_dev.detach().float().cpu().numpy()}
+    for k, v in tr.export_params().items():
+        out[k] = v.index_select(0, idx).float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(v, np.float32))
 
 
 class ClockSampler:
@@ -145,8 +174,8 @@ def reference_gpu_leg(path: str, config: str, n_gaussians: int, views: int, step
     baseline timed beside ours as the north_star asks -- never part of the product path.
     module 'b200': the SAME unchanged reference caller code linked against this library's host layer instead (the drop-in
     configuration a maintainer gets by switching the backend, INTEGRATION.md)."""
-    cmd = [sys.executable, os.path.join(ROOT, "tools", "ref_train.py"), "--module", module, "--path", path, "--config",
-           config, "--views", str(views), "--steps", str(max(2, min(steps, 4))), "--warmup", "2"]  # 2 warm-up steps: the
+    cmd = [sys.executable, "-B", os.path.join(ROOT, "tools", "ref_train.py"), "--module", module, "--path", path,
+           "--config", config, "--views", str(views), "--steps", str(max(2, min(steps, 4))), "--warmup", "2"]  # 2 warm-up steps: the
     # caching allocator needs them to hold a block for every per-view blob size (8 views, 4 blobs each)
     if n_gaussians:
         cmd += ["--n-gaussians", str(n_gaussians)]
@@ -338,6 +367,8 @@ def main():
         clocks.start()
     ms_step, launches = timed(step_resident, a.steps, a.warmup)
     clk = clocks.stop() if rank == 0 else {}
+    if a.dump_outputs and rank == 0:  # the later legs step the same parameters again
+        dump_last_step(tr, n, a.dump_outputs)
     ms_e2e, _ = timed(step_e2e, a.steps, max(1, a.warmup))
 
     # per-kernel timing for the roofline: a PROFILING pass outside the timed regions.  Every stage is bracketed by CUDA
@@ -441,8 +472,8 @@ def main():
         except Exception as e:
             line["drop_in"] = {"error": repr(e)}
         try:  # the EWA (fastgs) surface of this library on the same workload, op level (forward + backward per view)
-            r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "bench_fastgs.py"), a.config, "2", "2"],
-                               capture_output=True, text=True, timeout=300)
+            r = subprocess.run([sys.executable, "-B", os.path.join(ROOT, "tools", "bench_fastgs.py"), a.config, "2",
+                                "2"], capture_output=True, text=True, timeout=300)
             got = [l for l in r.stdout.splitlines() if l.startswith("{")]
             line["fastgs_surface"] = (json.loads(got[-1]) if got
                                       else {"error": (r.stderr or r.stdout).strip().splitlines()[-1][:300]})

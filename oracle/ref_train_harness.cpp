@@ -6,7 +6,7 @@
 //   src/training/kernels/ssim.cu + include/kernels/fused_ssim.cuh   fused_ssim (autograd)
 // on top of a fastgs backend chosen at LINK time (oracle/Makefile):
 //   ref_fastgs_torch   <- the reference's own fastgs objects (forward.cu, backward.cu, rasterization_api.cu, adam*.cu)
-//   b200_fastgs_torch  <- lichtfeld-studio_b200/libgsplat_backend_b200.so (this project's host layer, which exports the
+//   b200_fastgs_torch  <- oracle/_ref/libgsplat_backend_b200.so (this project's host layer, which exports the
 //                         same mangled fast_gs::rasterization::{forward,backward}_wrapper / fast_gs::optimizer symbols)
 // Both modules are the same object code above the backend boundary, so (a) the first is the "reference fastgs build"
 // training step timed beside ours, (b) the second proves that the reference's callers link and run against our

@@ -196,7 +196,7 @@ def require_all():
     """On a box with a CUDA device the reference builds MUST be present: a missing oracle/_ref/*.so would silently turn
     every 'vs the unmodified reference' assertion into a no-op (VERDICT r1, weak #3)."""
     import glob
-    missing = [n for n in ("libgsplat_ref.so", "libfastgs_ref.so", "libtorch_impl_ref.so")
+    missing = [n for n in ("libgsplat_ref.so", "libfastgs_ref.so", "libtorch_impl_ref.so", "libgsplat_backend_b200.so")
                if not os.path.exists(os.path.join(_REF, n))]
     for mod in ("ref_fastgs_torch", "b200_fastgs_torch"):
         if not glob.glob(os.path.join(_REF, mod + "*.so")):
@@ -257,6 +257,10 @@ def fastgs_torch_module(which="ref"):
         return sys.modules[name]
     hits = glob.glob(os.path.join(_REF, name + "*.so"))
     assert hits, f"oracle/_ref/{name}*.so missing"
+    if which == "b200":
+        # the host layer the module links against, loaded by path so that the module resolves it by its soname whatever
+        # run path the module was linked with
+        C.CDLL(os.path.join(_REF, "libgsplat_backend_b200.so"), mode=C.RTLD_GLOBAL)
     spec = importlib.util.spec_from_file_location(name, hits[0])
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)

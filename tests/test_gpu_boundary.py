@@ -4,7 +4,7 @@ oracle/ref_train_harness.cpp holds the reference's own callers compiled unchange
 (fast_rasterizer_autograd.cpp), SphericalHarmonicsFunction / fully_fused_projection_with_ut / GUTRasterizationFunction
 (rasterizer_autograd.cpp), FusedAdam (fused_adam.cpp), fused_ssim (ssim.cu) -- and is linked twice:
     ref_fastgs_torch   on the reference's own fastgs + gsplat CUDA objects
-    b200_fastgs_torch  on lichtfeld-studio_b200/libgsplat_backend_b200.so (this project's host layer)
+    b200_fastgs_torch  on oracle/_ref/libgsplat_backend_b200.so (this project's host layer)
 Every test runs the same call through both modules and compares: all 10 gsplat:: ops, forward_wrapper /
 backward_wrapper, adam_step_wrapper go through the host layer on the GPU (so libgsplat_backend_b200.so shows up in the
 driver's native_so_loaded), with the reference's callers above it bit-for-bit the same object code.

@@ -8,7 +8,7 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "lichtfeld-studio_b200", "libgsplat_backend_b200.so")
+LIB = os.path.join(ROOT, "oracle", "_ref", "libgsplat_backend_b200.so")
 
 
 def test_reference_symbol_fixture_is_complete():

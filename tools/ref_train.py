@@ -12,7 +12,6 @@ Prints one JSON line: views/s (CUDA events on the current stream, steps brackete
 plausibility check of the first forward (finite image, n_buckets consistent).  TEST / BENCH INFRASTRUCTURE ONLY."""
 import argparse
 import glob
-import importlib.util
 import json
 import os
 import sys
@@ -21,7 +20,8 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+import ref_libs  # noqa: E402
 from lichtfeld_studio_b200 import scene as S  # noqa: E402
 
 LRS = [0.00016, 0.0025, 0.0025 / 20, 0.005, 0.001, 0.05]  # eval/default_optimization_params.json, FusedAdam group order
@@ -29,13 +29,9 @@ LRS = [0.00016, 0.0025, 0.0025 / 20, 0.005, 0.001, 0.05]  # eval/default_optimiz
 
 def load_module(which: str):
     name = {"ref": "ref_fastgs_torch", "b200": "b200_fastgs_torch"}[which]
-    hits = glob.glob(os.path.join(ROOT, "oracle", "_ref", name + "*.so"))
-    if not hits:
+    if not glob.glob(os.path.join(ROOT, "oracle", "_ref", name + "*.so")):
         raise FileNotFoundError(f"oracle/_ref/{name}*.so not built (make -C oracle fastgs_torchmod)")
-    spec = importlib.util.spec_from_file_location(name, hits[0])
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+    return ref_libs.fastgs_torch_module(which)
 
 
 def scene_tensors(sc, dev):
